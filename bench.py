@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the GenPercept one-step hot path (BASELINE.json metric: images/sec at 768x768 depth).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -25,6 +25,10 @@ sample of the batch), with the thread count chosen by a probe at the benched siz
   1  one 512x512 depth image (the reference's CPU plumbing case)      3  normal 768x768, 8 / rank, all-gather of the maps
   2  depth 768x768, batch 8 / GPU (default)                           4  DPT readout 768x768, 4 / rank
   5  depth, batch 1, resolution sweep 384 / 512 / 768 / 1024 (one line; `sweep` holds the four points)
+
+--dump-outputs DIR writes what the last device-resident timed step returned (rank 0's fp32 maps, [B, C, H, W]) to
+DIR/prediction.npy, so that two builds can be compared output for output: inputs and weights are seeded, so the same
+arguments give the same inputs.  Maps larger than 64 MB are thinned to every k-th element of the flattened array.
 """
 import argparse
 import json
@@ -46,6 +50,7 @@ from genpercept_b200 import weights as W  # noqa: E402
 
 METRIC = "images/sec at 768x768 depth"
 UNIT = "images/s"
+DUMP_LIMIT = 64 << 20
 
 
 def text_embed():
@@ -107,6 +112,18 @@ class ClockSampler:
         busy = [s for s, p in zip(sm, pw) if p > 300] or sm
         return {"sm_mhz": statistics.median(busy) if busy else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(d, arrays):
+    """arrays: name -> float32 / float64 numpy array; each one thinned to a fixed stride to stay under DUMP_LIMIT in all."""
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    stride = -(-total // DUMP_LIMIT)
+    for name, a in arrays.items():
+        if stride > 1:
+            a = np.ascontiguousarray(a.reshape(-1)[::stride])
+            print(f"bench: {name} thinned to every {stride}th element ({a.size} values)", file=sys.stderr)
+        np.save(os.path.join(d, f"{name}.npy"), a)
 
 
 def best_thread_count(p, cores, res, mode="depth"):
@@ -207,7 +224,13 @@ def main():
     ap.add_argument("--ref-res", type=int, default=None, help="CPU arm: image size (default: the benched size)")
     ap.add_argument("--cuda-graph", action="store_true")
     ap.add_argument("--ops-json", default=None, help="write the per-op timing table here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the maps the last timed step computed to DIR/prediction.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     for k, v in CONFIGS[args.config].items():
         if k != "sweep" and getattr(args, k, None) is None:
             setattr(args, k, v)
@@ -250,7 +273,8 @@ def main():
         return float(t.item())
 
     def measure(B, R, steps, warmup, sampler=None):
-        """-> (ms device-resident, ms end to end) for `steps` steps of B images R x R, max over ranks."""
+        """-> (ms device-resident, ms end to end, host copy of the last device-resident step's maps or None) for `steps`
+        steps of B images R x R, max over ranks."""
         g = torch.Generator().manual_seed(1002 + rank)
         host_in = [torch.randint(0, 256, (B, 3, R, R), generator=g, dtype=torch.uint8).pin_memory() for _ in range(2)]
         dev_in = [h.cuda() for h in host_in]
@@ -266,11 +290,12 @@ def main():
         # ---- device-resident timing (value): the last kernel writes straight into dev_out
         barrier()
         e0.record()
-        for i in range(steps):
-            eng.infer(dev_in[i % 2], out_channels=C, out=dev_out)
+        for i in range(steps):      # the last step always takes dev_in[0]: --dump-outputs does not depend on --steps
+            eng.infer(dev_in[(steps - 1 - i) % 2], out_channels=C, out=dev_out)
         e1.record()
         barrier()
         ms_dev = max_over_ranks(e0.elapsed_time(e1))
+        last = dev_out.cpu().numpy() if args.dump_outputs else None       # outside both timed regions
         # ---- end to end through the public API with host buffers (e2e)
         barrier()
         e0.record()
@@ -288,11 +313,11 @@ def main():
         e1.record()
         barrier()
         ms_e2e = max_over_ranks(e0.elapsed_time(e1))
-        return ms_dev, ms_e2e
+        return ms_dev, ms_e2e, last
 
     sampler = ClockSampler(local) if rank == 0 else None
     B, R = args.batch, args.res
-    ms_dev, ms_e2e = measure(B, R, args.steps, args.warmup, sampler)
+    ms_dev, ms_e2e, last = measure(B, R, args.steps, args.warmup, sampler)
     clocks = sampler.stop() if rank == 0 else None
     info = eng.plan_info()
 
@@ -300,7 +325,7 @@ def main():
     if args.config == 5:            # resolution sweep, batch 1 (the headline stays the 768x768 point measured above)
         sweep = []
         for r in CONFIGS[5]["sweep"]:
-            d, e = (ms_dev, ms_e2e) if r == R else measure(1, r, args.steps, args.warmup)
+            d, e = (ms_dev, ms_e2e) if r == R else measure(1, r, args.steps, args.warmup)[:2]
             fl = FL.single_infer_flops(r, r, args.readout)
             sweep.append({"res": r, "ms_per_image": d / args.steps, "images_per_s": world * args.steps / (d / 1000.0),
                           "e2e_images_per_s": world * args.steps / (e / 1000.0),
@@ -386,6 +411,8 @@ def main():
         if sweep is not None:
             out["sweep"] = sweep
         print(json.dumps(out))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"prediction": last})
     if world > 1:
         dist.destroy_process_group()
 

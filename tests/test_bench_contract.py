@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -32,8 +33,8 @@ def test_reference_arm_line_on_cpu():
 
 
 @pytest.mark.gpu
-def test_engine_arm_line_on_gpu():
-    j = _run(["--steps", "3", "--warmup", "3", "--batch", "1", "--res", "128", "--ref-res", "64"])
+def test_engine_arm_line_on_gpu(tmp_path):
+    j = _run(["--steps", "3", "--warmup", "3", "--batch", "1", "--res", "128", "--ref-res", "64", "--dump-outputs", str(tmp_path)])
     assert BASE_KEYS <= set(j) and "impl" not in j or j.get("impl") == "ours"
     assert j["n_gpus"] == 1 and j["steps"] == 3 and j["warmup"] >= 3 and j["scaling"] == "weak" and j["dtype"] == "f16"
     assert j["value"] > 0 and j["e2e"]["value"] > 0 and j["gpu_launches"] > 0
@@ -42,6 +43,27 @@ def test_engine_arm_line_on_gpu():
     assert r["bound"] == "tensor" and r["unit"] == "TFLOP/s" and 0 < r["frac"] and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
     assert {"value", "unit", "cores", "kind", "sample"} <= set(j["cpu_baseline"])
     assert "workload" in j["config"] and "sm_mhz" in j["clocks"]
+    pred = np.load(tmp_path / "prediction.npy")             # the maps of the last timed step
+    assert pred.shape == (1, 1, 128, 128) and pred.dtype == np.float32 and 0 <= pred.min() and pred.max() <= 1
+
+
+def test_dump_outputs_stays_under_the_size_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 4096)
+    small, big = np.arange(512, dtype=np.float32), np.arange(2048, dtype=np.float64)
+    bench.dump_outputs(str(tmp_path / "a"), {"small": small})
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small)
+    bench.dump_outputs(str(tmp_path / "b"), {"small": small, "big": big})      # 2048 + 16384 bytes: every 5th element
+    got = {n: np.load(tmp_path / "b" / f"{n}.npy") for n in ("small", "big")}
+    assert np.array_equal(got["small"], small[::5]) and np.array_equal(got["big"], big[::5])
+    assert sum(v.nbytes for v in got.values()) <= 4096
+
+
+def test_steps_must_be_positive():
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=300, cwd=ROOT)
+    assert p.returncode != 0 and "--steps" in p.stderr
 
 
 def test_reference_arm_under_torchrun_prints_one_line():

@@ -1,7 +1,7 @@
 """Two-GPU NCCL test of parallel.sharded_infer with the real engine under torchrun (SURVEY.md 8e): every rank runs its
 shard of the batch on its own replica; the stacked result on every rank equals the single-GPU result bit for bit (images
 are independent; the per-image arithmetic does not depend on which rank runs it, only on the plan's batch size, so both
-sides use per-rank batch 2).  Needs 2 GPUs (`gpurun --gpus 2`); skipped on the 1-GPU box."""
+sides use per-rank batch 2).  Needs 2 GPUs; skipped on a machine with one."""
 import os
 import subprocess
 import sys
@@ -40,7 +40,7 @@ sys.exit(0 if ok else 1)
 '''
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_sharded_infer_two_gpus_nccl(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(WORKER)

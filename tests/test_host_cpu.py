@@ -85,14 +85,13 @@ def test_dropin_seeds_the_reference_import_path(tmp_path):
                        env=dict(os.environ, PYTHONPATH=root), capture_output=True, text=True, timeout=300)
     assert p.returncode == 0, p.stderr[-2000:]
     assert "genpercept_b200.pipeline genpercept_b200.pipeline reference util ['--mode', 'depth']" in p.stdout
-    ref = "/root/reference"
-    if os.path.isdir(os.path.join(ref, "genpercept")):        # and against the real checkout where it exists (not on the GPU box)
-        code = ("import genpercept_b200.dropin as d; d.install(); from genpercept import GenPerceptPipeline as P; "
-                "import genpercept; print(P.__module__, genpercept.__file__)")
-        q = subprocess.run([sys.executable, "-c", code], cwd=ref, env=dict(os.environ, PYTHONPATH=root), capture_output=True,
-                           text=True, timeout=300)
-        assert q.returncode == 0, q.stderr[-2000:]
-        assert "genpercept_b200.pipeline /root/reference/genpercept/__init__.py" in q.stdout
+    # the in-process route (dropin.install()) resolves the same package from the working directory
+    code = ("import genpercept_b200.dropin as d; d.install(); from genpercept import GenPerceptPipeline as P; "
+            "import genpercept; print(P.__module__, genpercept.__file__)")
+    q = subprocess.run([sys.executable, "-c", code], cwd=tmp_path, env=dict(os.environ, PYTHONPATH=root), capture_output=True,
+                       text=True, timeout=300)
+    assert q.returncode == 0, q.stderr[-2000:]
+    assert f"genpercept_b200.pipeline {pkg / '__init__.py'}" in q.stdout
 
 
 def test_tile_shape_policy():

@@ -102,24 +102,24 @@ def test_cross_attention_two_token_closed_form(synth_state, text_embed):
     torch.testing.assert_close(out, ref, atol=2e-5, rtol=1e-4)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="needs the reference tree (build container only)")
-def test_upsample2d_matches_the_reference_vendored_class():
-    """/root/reference/genpercept/models/dpt_head.py:92-210 vendors diffusers' ``Upsample2D`` — the one block of the
+def test_upsample2d_matches_the_reference_vendored_class(golden_dir):
+    """genpercept/models/dpt_head.py:92-210 in the reference vendors diffusers' ``Upsample2D`` — the one block of the
     UNet / VAE graphs whose source IS in the reference tree.  oracle.blocks.Upsample2D (used by every up block of both
-    graphs) must match it, including the explicit-size path diffusers takes when a level has an odd extent."""
+    graphs) must match it bit for bit, including the explicit-size path diffusers takes when a level has an odd extent.
+    The reference's results are stored as digests (tests/golden/make_golden_reference.py); input and weights are
+    integer-valued, so the float32 result is exact on any machine."""
     import importlib.util
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import make_golden                      # installs the 2-symbol diffusers shim
-    make_golden.load_reference_dpt()
-    ref_mod = sys.modules["ref_dpt_head"]
+    spec = importlib.util.spec_from_file_location("mkref", os.path.join(golden_dir, "make_golden_reference.py"))
+    mk = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mk)
+    ref = np.load(os.path.join(golden_dir, "reference_glue.npz"))
     from oracle.blocks import Upsample2D
-    torch.manual_seed(3)
-    ref = ref_mod.Upsample2D(24, use_conv=True).eval()
+    x, w, b = mk.upsample_case()
     mine = Upsample2D(24).eval()
-    mine.conv.load_state_dict(ref.conv.state_dict())
-    x = torch.randn(2, 24, 7, 9)
+    mine.conv.load_state_dict({"weight": w, "bias": b})
     with torch.no_grad():
-        assert torch.equal(mine(x), ref(x))
-        for size in ((13, 17), (14, 18), (13, 18)):
-            assert torch.equal(mine(x, size), ref(x, output_size=size))
+        for size in mk.UPSAMPLE_SIZES:
+            y = mine(x) if size is None else mine(x, size)
+            key = "none" if size is None else f"{size[0]}x{size[1]}"
+            assert tuple(y.shape) == tuple(ref[f"upsample_{key}_shape"]), key
+            assert mk.digest(y) == str(ref[f"upsample_{key}_sha256"]), key

@@ -1,253 +1,89 @@
-"""Pins the oracle's orchestration (oracle/pipeline.py) against the REFERENCE'S OWN ``GenPerceptPipeline.single_infer`` /
-``encode_rgb`` / ``decode_pred`` (/root/reference/genpercept/genpercept_pipeline.py:375-526), executed here:
+"""Pins the oracle's orchestration (oracle/pipeline.py) and the oracle's UNet dataflow against the REFERENCE'S OWN code:
+``GenPerceptPipeline.single_infer`` / ``encode_rgb`` / ``decode_pred`` (genpercept/genpercept_pipeline.py:375-526),
+``CustomUNet2DConditionModel.forward`` (genpercept/models/custom_unet.py:34-427), ``DDIMSchedulerCustomized``, the host
+image helpers and the first release's pipeline.
 
-the reference module is imported through a minimal ``diffusers`` / ``matplotlib`` shim (base classes and type names only:
-diffusers itself is not installable here) and instantiated with the oracle's VAE / UNet modules and one-step scheduler
-behind thin adapters, plus the reference's own DPT head class.  Everything between those modules — latent scaling, the
-mean half of the moments, the scheduler call and ``pred_original_sample``, ``/ scale`` + post_quant_conv + decoder, the
-channel mean, clip and shift, the DPT feature order and min-max — is then the reference's code, not a restatement.
-(What stays unpinned is the inside of the diffusers blocks; see oracle/__init__.py.)  Build container only."""
-import importlib
+tests/golden/make_golden_reference.py ran the reference's code around THIS package's modules (the oracle's VAE / UNet /
+scheduler behind thin adapters, the reference's own DPT head class) and stored what it computed in
+tests/golden/reference_glue.npz.  Everything between those modules — latent scaling, the mean half of the moments, the
+scheduler call and ``pred_original_sample``, ``/ scale`` + post_quant_conv + decoder, the channel mean, clip and shift,
+the DPT feature order and min-max, the skip stack and ``upsample_size`` forwarding — was the reference's code; here the
+oracle runs the same modules on the same weights and inputs and must land on the stored results.  Both sides run in
+float64 so that the tolerances below do not depend on this machine's float32 summation order.
+(What stays unpinned is the inside of the diffusers blocks; see oracle/__init__.py.)"""
+import importlib.util
 import os
-import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference tree (build container only)")
 
-
-def _install_shims():
-    import torch.nn as nn
-    if "diffusers" not in sys.modules or not hasattr(sys.modules["diffusers"], "DiffusionPipeline"):
-        d = sys.modules.get("diffusers") or types.ModuleType("diffusers")
-
-        class DiffusionPipeline:
-            def __init__(self):
-                self._cfg = {}
-
-            def register_modules(self, **kw):
-                for k, v in kw.items():
-                    setattr(self, k, v)
-
-            def register_to_config(self, **kw):
-                self._cfg.update(kw)
-
-            @property
-            def device(self):
-                return torch.device("cpu")
-
-            @property
-            def dtype(self):
-                return torch.float32
-
-        for name in ("AutoencoderKL", "DDIMScheduler", "LCMScheduler", "UNet2DConditionModel"):
-            setattr(d, name, type(name, (), {}))
-        d.DiffusionPipeline = DiffusionPipeline
-        du = sys.modules.get("diffusers.utils") or types.ModuleType("diffusers.utils")
-        du.BaseOutput = type("BaseOutput", (), {})
-        du.USE_PEFT_BACKEND = True
-        dm = sys.modules.get("diffusers.models") or types.ModuleType("diffusers.models")
-        dl = sys.modules.get("diffusers.models.lora") or types.ModuleType("diffusers.models.lora")
-        dl.LoRACompatibleConv = nn.Conv2d
-        d.utils, d.models, dm.lora = du, dm, dl
-        sys.modules.update({"diffusers": d, "diffusers.utils": du, "diffusers.models": dm, "diffusers.models.lora": dl})
-    if "matplotlib" not in sys.modules:
-        m = types.ModuleType("matplotlib")
-        mp = types.ModuleType("matplotlib.pyplot")
-        m.pyplot = mp
-        sys.modules.update({"matplotlib": m, "matplotlib.pyplot": mp})
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-
-
-class _UNetAdapter:
-    def __init__(self, unet):
-        self.unet = unet
-
-    def __call__(self, x, t, encoder_hidden_states=None, return_feature=False):
-        t = torch.as_tensor(t).reshape(-1)[:1]
-        out = self.unet(x, t, encoder_hidden_states, return_feature=return_feature)
-        return types.SimpleNamespace(multi_level_feats=out) if return_feature else types.SimpleNamespace(sample=out)
-
-
-class _SchedulerAdapter:
-    beta_start = 1
-    beta_end = 1
-
-    def __init__(self, s):
-        self.s = s
-
-    def set_timesteps(self, n, device=None):
-        self.timesteps = self.s.set_timesteps(n)
-
-    def step(self, model_output, t, sample, generator=None):
-        prev, x0 = self.s.step(model_output, int(t), sample)
-        return types.SimpleNamespace(prev_sample=prev, pred_original_sample=x0)
+@pytest.fixture(scope="module")
+def mk(golden_dir):
+    spec = importlib.util.spec_from_file_location("make_golden_reference", os.path.join(golden_dir, "make_golden_reference.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
 
 
 @pytest.fixture(scope="module")
-def ref_pipeline_cls():
-    _install_shims()
-    return importlib.import_module("genpercept.genpercept_pipeline")
+def ref(golden_dir):
+    return np.load(os.path.join(golden_dir, "reference_glue.npz"))
 
 
-def test_single_infer_glue_matches_the_reference(ref_pipeline_cls, synth_state, text_embed):
+def _close(mine, want, atol):
+    mine = mine.double()
+    want = torch.from_numpy(want).double()
+    assert mine.shape == want.shape, (tuple(mine.shape), tuple(want.shape))
+    assert torch.allclose(mine, want, atol=atol, rtol=0), float((mine - want).abs().max())
+
+
+def test_single_infer_glue_matches_the_reference(mk, ref, synth_state, text_embed):
     from oracle.pipeline import OraclePipeline
-    mod = ref_pipeline_cls
-    g = torch.Generator().manual_seed(21)
-    rgb = torch.rand((1, 3, 64, 64), generator=g) * 2 - 1
+    rgb = mk.glue_input().double()
     # VAE readout, 1- and 3-channel modes
-    op = OraclePipeline(synth_state, text_embed)
-    rp = mod.GenPerceptPipeline(unet=_UNetAdapter(op.unet), vae=op.vae, scheduler=_SchedulerAdapter(op.scheduler),
-                                text_encoder=None, tokenizer=None, genpercept_pipeline=True)
-    rp.text_embed = op.text_embed
+    op = OraclePipeline(synth_state, text_embed, dtype=torch.float64)
     for mode in ("depth", "normal"):
-        rp.mode = mode
-        with torch.no_grad():
-            ref = rp.single_infer(rgb, 1, None, False)
-        mine = op.single_infer(rgb, mode=mode)
-        assert ref.shape == mine.shape and torch.allclose(ref, mine, atol=1e-6, rtol=0), float((ref - mine).abs().max())
-    with torch.no_grad():
-        assert torch.allclose(rp.encode_rgb(rgb), op.encode_rgb(rgb), atol=1e-7)
+        _close(op.single_infer(rgb, mode=mode), ref[f"glue_{mode}"], 1e-6)
+    _close(op.encode_rgb(rgb), ref["glue_encode_rgb"], 1e-7)
     # --fix_timesteps: the reference feeds that timestep to the UNet instead of the scheduler's
-    with torch.no_grad():
-        ref = rp.single_infer(rgb, 1, None, False, fix_timesteps=7)
-    assert torch.allclose(ref, op.single_infer(rgb, mode="normal", fix_timesteps=7), atol=1e-6, rtol=0)
-    # DPT readout with the reference's own head class (isinstance check at genpercept_pipeline.py:475)
-    od = OraclePipeline(synth_state, text_embed, use_dpt=True)
-    head_mod = sys.modules["genpercept.models.dpt_head"]
-    # transformers >= 4.4x refuses ModelOutput subclasses that are not dataclasses; the reference's output container
-    # (dpt_head.py:24-49, written for an older transformers) is replaced by a plain attribute bag — no arithmetic involved
-    head_mod.DepthEstimatorOutput = lambda **kw: types.SimpleNamespace(**kw)
-    from transformers import DPTConfig
-    head = head_mod.DPTNeckHeadForUnetAfterUpsampleIdentity(
-        DPTConfig.from_pretrained(f"{REF}/hf_configs/dpt-sd2.1-unet-after-upsample-general")).eval()
-    head.load_state_dict(synth_state["dpt"], strict=True)
-    rd = mod.GenPerceptPipeline(unet=_UNetAdapter(od.unet), vae=od.vae, scheduler=_SchedulerAdapter(od.scheduler),
-                                text_encoder=None, tokenizer=None, customized_head=head, genpercept_pipeline=True)
-    rd.text_embed = od.text_embed
-    rd.mode = "depth"
-    with torch.no_grad():
-        ref = rd.single_infer(rgb, 1, None, False)
-    mine = od.single_infer(rgb, mode="depth")
-    assert ref.shape == mine.shape and torch.allclose(ref, mine, atol=2e-6, rtol=0), float((ref - mine).abs().max())
+    _close(op.single_infer(rgb, mode="normal", fix_timesteps=7), ref["glue_normal_fix_timesteps_7"], 1e-6)
+    del op
+    # DPT readout (the reference ran its own head class on the same weights)
+    od = OraclePipeline(synth_state, text_embed, use_dpt=True, dtype=torch.float64)
+    _close(od.single_infer(rgb, mode="depth"), ref["glue_dpt"], 2e-6)
 
 
-def _install_unet_shims():
-    import torch.nn as nn
-    _install_shims()
-    d = sys.modules["diffusers"]
-    d.UNet2DConditionModel = type("UNet2DConditionModel", (nn.Module,), {})
-    du = sys.modules["diffusers.utils"]
-    du.deprecate = lambda *a, **k: None
-    du.logging = types.SimpleNamespace(get_logger=lambda *a, **k: None)
-    du.scale_lora_layers = lambda *a, **k: None
-    du.unscale_lora_layers = lambda *a, **k: None
-    unets = types.ModuleType("diffusers.models.unets")
-    u2d = types.ModuleType("diffusers.models.unets.unet_2d_condition")
-    u2d.UNet2DConditionOutput = type("UNet2DConditionOutput", (), {})
-    sys.modules.update({"diffusers.models.unets": unets, "diffusers.models.unets.unet_2d_condition": u2d})
-
-
-def test_unet_dataflow_matches_the_reference_forward(synth_state, text_embed):
-    """/root/reference/genpercept/models/custom_unet.py:34-427 (the reference's own UNet forward: skip stack, the
-    `upsample_size` forwarding for odd extents, the DPT feature taps, conv_norm_out / conv_out) is executed here around
-    the ORACLE's blocks, attached to an instance of the reference class, and compared with oracle.unet's forward."""
-    import torch.nn as nn
-    _install_unet_shims()
-    spec = importlib.util.spec_from_file_location("ref_custom_unet", f"{REF}/genpercept/models/custom_unet.py")
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
+def test_unet_dataflow_matches_the_reference_forward(mk, ref, synth_state, text_embed):
+    """The reference's own UNet forward (skip stack, the `upsample_size` forwarding for odd extents, the DPT feature taps,
+    conv_norm_out / conv_out) was executed around the ORACLE's blocks, attached to an instance of the reference class;
+    oracle.unet's forward must give its output and (a fixed, seeded sample of) its feature maps."""
     from oracle.pipeline import OraclePipeline
-    ou = OraclePipeline(synth_state, text_embed).unet
-
-    class Down(nn.Module):
-        def __init__(self, blk, cross):
-            super().__init__()
-            self.blk, self.has_cross_attention = blk, cross
-
-        def forward(self, hidden_states, temb, encoder_hidden_states=None, **kw):
-            return self.blk(hidden_states, temb, encoder_hidden_states)
-
-    class Mid(nn.Module):
-        has_cross_attention = True
-
-        def __init__(self, blk):
-            super().__init__()
-            self.blk = blk
-
-        def forward(self, sample, emb, encoder_hidden_states=None, **kw):
-            return self.blk(sample, emb, encoder_hidden_states)
-
-    class Up(nn.Module):
-        def __init__(self, blk):
-            super().__init__()
-            self.blk, self.has_cross_attention, self.resnets = blk, blk.attentions is not None, blk.resnets
-
-        def forward(self, hidden_states, temb, res_hidden_states_tuple, encoder_hidden_states=None, upsample_size=None, **kw):
-            return self.blk(hidden_states, res_hidden_states_tuple, temb, encoder_hidden_states, upsample_size)
-
-    class TimeEmb(nn.Module):
-        def __init__(self, m):
-            super().__init__()
-            self.m = m
-
-        def forward(self, t_emb, cond=None):
-            return self.m(t_emb)
-
-    ru = mod.CustomUNet2DConditionModel()
-    ru.num_upsamplers = 3
-    ru.config = types.SimpleNamespace(center_input_sample=False, class_embed_type=None, addition_embed_type=None,
-                                      class_embeddings_concat=False, encoder_hid_dim_type=None)
-    ru.class_embedding = ru.time_embed_act = ru.encoder_hid_proj = None
-    ru.time_proj, ru.time_embedding = ou.time_proj, TimeEmb(ou.time_embedding)
-    ru.conv_in, ru.conv_norm_out, ru.conv_act, ru.conv_out = ou.conv_in, ou.conv_norm_out, nn.SiLU(), ou.conv_out
-    ru.down_blocks = nn.ModuleList([Down(b, i < 3) for i, b in enumerate(ou.down_blocks)])
-    ru.mid_block = Mid(ou.mid_block)
-    ru.up_blocks = nn.ModuleList([Up(b) for b in ou.up_blocks])
-    ru.eval()
-    g = torch.Generator().manual_seed(4)
-    ctx = text_embed.float().reshape(1, -1, 1024)
-    for h, w in ((8, 8), (9, 11), (12, 10)):                    # multiples of 8, odd extents, 8 does not divide
-        x = torch.randn((1, 4, h, w), generator=g)
+    ou = OraclePipeline(synth_state, text_embed, dtype=torch.float64).unet
+    ctx = text_embed.double().reshape(1, -1, 1024)
+    for (h, w), x in zip(mk.UNET_SIZES, mk.unet_inputs()):
+        key = f"unet_{h}x{w}"
         with torch.no_grad():
-            ref = ru(x, 1, ctx)
-            mine = ou(x, torch.tensor([1]), ctx)
-            assert torch.allclose(ref.sample, mine, atol=1e-6, rtol=0), (h, w, float((ref.sample - mine).abs().max()))
-            rf = ru(x, torch.tensor([1]), ctx, return_feature=True).multi_level_feats
-            mf = ou(x, torch.tensor([1]), ctx, return_feature=True)
-            assert len(rf) == len(mf) == 4
-            for a, b in zip(rf, mf):
-                assert a.shape == b.shape and torch.allclose(a, b, atol=1e-5, rtol=0)
+            _close(ou(x.double(), torch.tensor([1]), ctx), ref[f"{key}_sample"], 1e-6)
+            mf = ou(x.double(), torch.tensor([1]), ctx, return_feature=True)
+        assert len(mf) == 4
+        for i, f in enumerate(mf):
+            assert tuple(f.shape) == tuple(ref[f"{key}_feat{i}_shape"]), (key, i)
+            idx = torch.from_numpy(ref[f"{key}_feat{i}_idx"].astype(np.int64))
+            _close(f.reshape(-1)[idx], ref[f"{key}_feat{i}_val"], 1e-5)
 
 
-def test_scheduler_constants_match_the_reference_class():
-    """/root/reference/src/customized_modules/ddim.py:144-217 (DDIMSchedulerCustomized.__init__ — the part
-    of the scheduler that IS in the reference tree; set_timesteps / step are diffusers') instantiated from the
-    reference's own hf_configs/scheduler_beta_1.0_1.0/scheduler_config.json, against oracle.scheduler.DDIMOneStep."""
-    import json
-    _install_shims()
-    d = sys.modules["diffusers"]
-    d.DDIMScheduler = getattr(d, "DDIMScheduler", type("DDIMScheduler", (), {}))
-    d.DDPMScheduler = type("DDPMScheduler", (), {})
-    cu = types.ModuleType("diffusers.configuration_utils")
-    cu.ConfigMixin = type("ConfigMixin", (), {})
-    cu.register_to_config = lambda f: f
-    sys.modules["diffusers.configuration_utils"] = cu
-    spec = importlib.util.spec_from_file_location("ref_ddim", f"{REF}/src/customized_modules/ddim.py")
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    cfg = json.load(open(f"{REF}/hf_configs/scheduler_beta_1.0_1.0/scheduler_config.json"))
-    kw = {k: v for k, v in cfg.items() if not k.startswith("_") and k != "skip_prk_steps"}
-    ref = mod.DDIMSchedulerCustomized(**kw)
+def test_scheduler_constants_match_the_reference_class(ref):
+    """src/customized_modules/ddim.py:144-217 (DDIMSchedulerCustomized.__init__ — the part of the scheduler that IS in
+    the reference tree; set_timesteps / step are diffusers') instantiated from the reference's own
+    hf_configs/scheduler_beta_1.0_1.0/scheduler_config.json, against oracle.scheduler.DDIMOneStep."""
     from oracle.scheduler import DDIMOneStep
     mine = DDIMOneStep()
-    assert torch.equal(ref.betas, mine.betas) and torch.equal(ref.alphas_cumprod, mine.alphas_cumprod)
-    assert torch.equal(ref.final_alpha_cumprod, mine.final_alpha_cumprod)
-    assert float(ref.alphas_cumprod[1]) == 0.0 and ref.init_noise_sigma == 1.0       # beta = 1: x_t carries no signal
+    assert torch.equal(torch.from_numpy(ref["sched_betas"]), mine.betas)
+    assert torch.equal(torch.from_numpy(ref["sched_alphas_cumprod"]), mine.alphas_cumprod)
+    assert torch.equal(torch.from_numpy(ref["sched_final_alpha_cumprod"]), mine.final_alpha_cumprod)
+    assert float(ref["sched_alphas_cumprod"][1]) == 0.0 and float(ref["sched_init_noise_sigma"]) == 1.0  # beta = 1
     # one DDIM step at the single timestep the pipeline uses (t = 1, leading spacing + offset 1): x0 = -v
     ts = mine.set_timesteps(1)
     assert ts.tolist() == [1]
@@ -257,57 +93,36 @@ def test_scheduler_constants_match_the_reference_class():
     assert torch.equal(x0, -v)
 
 
-def test_host_image_helpers_match_the_reference_functions():
+def test_host_image_helpers_match_the_reference_functions(mk, ref):
     """genpercept_b200.image_util (host mirror) and oracle.imgproc against the reference's own
-    genpercept/util/image_util.py: resize_max_res (:75-105), get_tv_resample_method (:108-119), chw2hwc (:66-72)."""
-    import numpy as np
-    _install_shims()
-    ref = importlib.import_module("genpercept.util.image_util")
+    genpercept/util/image_util.py: resize_max_res (:75-105, bit for bit), get_tv_resample_method (:108-119), chw2hwc
+    (:66-72)."""
     from genpercept_b200 import image_util as mine
     from oracle import imgproc as IP
-    g = torch.Generator().manual_seed(8)
-    x = torch.randint(0, 256, (1, 3, 90, 160), generator=g, dtype=torch.uint8)
-    for edge in (64, 128, 200):
-        r = ref.resize_max_res(x, edge)
-        assert torch.equal(mine.resize_max_res(x, edge), r)
+    x, c = mk.resize_case()
+    for edge in mk.RESIZE_EDGES:
+        r = mine.resize_max_res(x, edge)
+        assert tuple(r.shape) == tuple(ref[f"resize_{edge}_shape"])
+        assert mk.digest(r) == str(ref[f"resize_{edge}_sha256"]), edge
         assert tuple(r.shape[-2:]) == IP.resize_max_res_shape(90, 160, edge)
         d = np.abs(IP.resize_aa(x.numpy(), *r.shape[-2:]).astype(np.int32) - r.numpy().astype(np.int32))
         assert d.max() <= 1 and (d > 0).mean() <= 1e-3
     for m in ("bilinear", "bicubic", "nearest"):
-        assert mine.get_tv_resample_method(m) == ref.get_tv_resample_method(m)
-    with pytest.raises(ValueError):
+        assert mine.get_tv_resample_method(m).value == str(ref[f"resample_{m}"])
+    with pytest.raises(ValueError):                           # the reference raises too
         mine.get_tv_resample_method("lanczos")
-    with pytest.raises(ValueError):
-        ref.get_tv_resample_method("lanczos")
-    c = torch.rand((3, 4, 5), generator=g)
-    assert torch.equal(mine.chw2hwc(c), ref.chw2hwc(c)) and np.array_equal(mine.chw2hwc(c.numpy()), ref.chw2hwc(c.numpy()))
+    assert torch.equal(mine.chw2hwc(c), torch.from_numpy(ref["chw2hwc_tensor"]))
+    assert np.array_equal(mine.chw2hwc(c.numpy()), ref["chw2hwc_array"])
 
 
-def test_legacy_v1_pipeline_closed_form_matches(synth_state):
-    """/root/reference/GenPercept_v1/genpercept/pipeline_genpercept.py:263-354 — the first release hard-codes what the v2
-    scheduler collapses to (t = 1, pred_latent = -unet_pred, no scheduler object) and feeds the full 77-token padded
-    empty-prompt embedding (GenPercept_v1/empty_text_embed.npy).  Its single_infer around the oracle's modules must equal
-    the oracle run with that 77-token context (range [-1,1] there, [0,1] in v2)."""
-    import numpy as np
-    _install_shims()
-    v1_root = f"{REF}/GenPercept_v1"
-    spec = importlib.util.spec_from_file_location("genpercept_v1", f"{v1_root}/genpercept/__init__.py",
-                                                  submodule_search_locations=[f"{v1_root}/genpercept"])
-    pkg = importlib.util.module_from_spec(spec)
-    sys.modules["genpercept_v1"] = pkg
-    try:
-        spec.loader.exec_module(pkg)
-        mod = importlib.import_module("genpercept_v1.pipeline_genpercept")
-    except Exception as e:                                  # the v1 helpers may need packages that are not installed
-        pytest.skip(f"GenPercept_v1 package not importable here: {e!r}")
+def test_legacy_v1_pipeline_closed_form_matches(mk, ref, synth_state):
+    """GenPercept_v1/genpercept/pipeline_genpercept.py:263-354 — the first release hard-codes what the v2 scheduler
+    collapses to (t = 1, pred_latent = -unet_pred, no scheduler object) and feeds the full 77-token padded empty-prompt
+    embedding (GenPercept_v1/empty_text_embed.npy, stored with the result).  Its single_infer around the oracle's modules
+    must equal the oracle run with that 77-token context (range [-1,1] there, [0,1] in v2)."""
     from oracle.pipeline import OraclePipeline
-    te = torch.from_numpy(np.load(f"{v1_root}/empty_text_embed.npy").astype(np.float32))[None]     # [1, 77, 1024]
-    op = OraclePipeline(synth_state, te)
-    p1 = mod.GenPerceptPipeline(unet=_UNetAdapter(op.unet), vae=op.vae, empty_text_embed=te)
-    g = torch.Generator().manual_seed(31)
-    rgb = torch.rand((1, 3, 64, 64), generator=g) * 2 - 1
-    with torch.no_grad():
-        ref = p1.single_infer(rgb, mode="depth")
-    mine = op.single_infer(rgb, mode="depth") * 2.0 - 1.0
-    # (x + 1) / 2 * 2 - 1 and the different place of the channel mean cost a few fp32 ulps of values up to 1
-    assert ref.shape == mine.shape and torch.allclose(ref, mine, atol=2e-5, rtol=0), float((ref - mine).abs().max())
+    te = torch.from_numpy(ref["v1_empty_text_embed"].astype(np.float32))[None]       # [1, 77, 1024]
+    op = OraclePipeline(synth_state, te, dtype=torch.float64)
+    mine = op.single_infer(mk.glue_input(31).double(), mode="depth") * 2.0 - 1.0
+    # (x + 1) / 2 * 2 - 1 and the different place of the channel mean cost a few ulps of values up to 1
+    _close(mine, ref["v1_depth"], 2e-5)
