@@ -15,10 +15,6 @@ namespace gp {
 size_t Arena::alloc(size_t bytes) {
   bytes = (bytes + 1023) & ~size_t(1023);
   if (bytes == 0) bytes = 1024;
-  // Experiment (GP_ARENA_SKEW=<KiB>): the big VAE tensors are exact multiples of 2^27 bytes, so the input, residual and
-  // output streams of one convolution can sit a power of two apart; a per-allocation skew de-aligns them.
-  static const size_t skew = std::getenv("GP_ARENA_SKEW") ? (size_t)std::atoi(std::getenv("GP_ARENA_SKEW")) * 1024 : 0;
-  if (skew && bytes >= (size_t(1) << 24)) bytes += skew * (1 + (nalloc_++ % 7));
   for (size_t i = 0; i < blks_.size(); ++i) {
     if (blks_[i].free && blks_[i].size >= bytes) {
       if (blks_[i].size > bytes) {
@@ -115,12 +111,10 @@ static int choose_bn(int cout, int force) {
   // Cout = 320 / 640 (the SD-2.1 UNet's first two levels): an exact divisor (160) is not a multiple of 64 and forces the
   // direct epilogue (16-byte stores at a 2*Cout-byte stride, per-thread residual rows, no GroupNorm statistics).  A
   // multiple of 64 keeps the staged TMA-store epilogue even if the last N tile is partly empty: 640 = 5 x 128 exactly,
-  // 320 -> 2 x 192 (64 idle columns).  GP_BN_POLICY=0 restores the divisor rule (A/B switch).
-  static const int policy = std::getenv("GP_BN_POLICY") ? std::atoi(std::getenv("GP_BN_POLICY")) : 1;
-  if (policy && (cout % 64) == 0) {
+  // 320 -> 2 x 192 (64 idle columns).
+  if ((cout % 64) == 0) {
     for (int bn : {256, 192, 128})
       if (cout % bn == 0) return bn;
-    if (policy == 2) return 128;
     int best = 256, best_pad = 1 << 30;
     for (int bn : {256, 192, 128}) {
       const int pad = ceil_div(cout, bn) * bn - cout;
@@ -151,12 +145,11 @@ static void choose_tile(int gw, int gh, int rows, int* tw, int* th, int* shift) 
 // 2560 -> 1280 conv on 8 x 12 x 12 pixels moves 796 MB with BN = 256 and 1062 MB with BN = 128: 152 vs 210 us, although
 // BN = 128 doubles the number of busy SMs; at batch 1 the same level has 2 M tiles, BN = 256 keeps 10 SMs busy for 61 us
 // and BN = 64 runs 40 tiles in ~25 us).  A candidate replaces the default only for a predicted gain above 10 %, so
-// every layer with many waves stays where choose_bn put it.  GP_TILE_MODEL=0: off (A/B switch).
+// every layer with many waves stays where choose_bn put it.
 struct TileShape { int bn, mt; };
 template <class MTilesFn>
 static TileShape choose_tile_shape(int cout, double k_elems, int num_sms, TileShape dflt, MTilesFn mtiles_of) {
-  static const bool off = [] { const char* e = std::getenv("GP_TILE_MODEL"); return e && e[0] == '0'; }();
-  if (off || cout % 64 != 0 || cout < 128) return dflt;
+  if (cout % 64 != 0 || cout < 128) return dflt;
   auto cost = [&](TileShape t) {
     const double tiles = (double)mtiles_of(t.mt) * ceil_div(cout, t.bn);
     const double waves = std::ceil(tiles / num_sms);
@@ -209,7 +202,7 @@ static void finalize_or_throw(IgemmParams* p, const std::string& name) {
 // operand fetch, which already uses the SM's whole shared-memory bandwidth on these layers: no net gain (DESIGN.md 4.1).
 static bool gn_fusable(const ConvArgs& a, bool split) {
   const char* on = std::getenv("GP_GN_FUSE");        // read at plan time (tests toggle it)
-  const bool off = on == nullptr || on[0] == '0' || std::getenv("GP_NO_PATCH") != nullptr;
+  const bool off = on == nullptr || on[0] == '0';
   if (off || split || a.mode != 0 || a.ks != 3 || a.srcs.size() != 1 || a.sc.size() > 1) return false;
   const T4& s = a.srcs[0];
   if ((s.W % 128) || (s.C % 64) || (!a.sc.empty() && (a.sc[0].C % 64))) return false;
@@ -268,16 +261,11 @@ void Builder::conv(const std::string& name, const ConvArgs& a) {
                    &bn_pre, &mt_pre);
   }
   const bool is_geglu = (a.flags & IG_GEGLU) != 0;
-  const bool staged = !a.out_f32 && std::getenv("GP_DIRECT_EPILOGUE") == nullptr &&
-                      (is_geglu ? (std::getenv("GP_STAGED_GEGLU") != nullptr && !split_ &&   // measured slower than the direct GEGLU stores (r1g)
-                                   Cout == 2 * a.out.C && (Cout % 128) == 0 && (bn_pre % 128) == 0)
-                                : (Cout == a.out.C && (Cout % 64) == 0 && (bn_pre % 64) == 0));
-  // GP_STATS: 0 = never fuse the GroupNorm partial sums into conv epilogues, 1 = always (default), 2 = everywhere
-  // except the patch-resident layers (whose main loop runs at the tensor-pipe limit, so the epilogue is critical)
-  static const int stats_mode = std::getenv("GP_STATS") ? std::atoi(std::getenv("GP_STATS")) : 1;
+  // GEGLU keeps the direct epilogue: a staged GEGLU epilogue measured slower than the direct stores (r1g, r2p)
+  const bool staged = !a.out_f32 && !is_geglu && Cout == a.out.C && (Cout % 64) == 0 && (bn_pre % 64) == 0;
   const bool patch_eligible = gn_fused || (staged && a.mode == 0 && a.ks == 3 && a.srcs.size() == 1 && a.sc.empty() && mt_pre == 2 &&
-                                           (W % 128) == 0 && (H % 2) == 0 && !split_ && std::getenv("GP_NO_PATCH") == nullptr);
-  bool emit_stats = a.want_stats && staged && !is_geglu && Cout <= 512 && stats_mode != 0 && !(stats_mode == 2 && patch_eligible) && !split_;
+                                           (W % 128) == 0 && (H % 2) == 0 && !split_);
+  bool emit_stats = a.want_stats && staged && Cout <= 512 && !split_;
   if (emit_stats && tokens_mode && ((long long)H * W) % (128 * mt_pre) != 0) emit_stats = false;
   size_t stats_off = 0;
   const size_t stats_bytes = (size_t)N * num_sms * Cout * 2 * sizeof(float);
@@ -435,9 +423,8 @@ void Builder::conv(const std::string& name, const ConvArgs& a) {
       }
     }
     // the residual has the output's shape and addressing: same maps over its base
-    if (a.res1 && !a.res2 && !(a.flags & IG_GEGLU) && !split_ && std::getenv("GP_NO_RES_TMA") == nullptr) {
+    if (a.res1 && !a.res2 && !split_) {
       p.res_tma = 1;
-      p.res_prefetch = std::getenv("GP_NO_RES_PREFETCH") == nullptr ? 1 : 0;
       const void* rb = ptr(*a.res1);
       if (tokens) {
         const long long ntok = (long long)N * H * W;
@@ -475,10 +462,7 @@ void Builder::conv(const std::string& name, const ConvArgs& a) {
     if (gn_fused) {
       p.gn_ss = gn_ss;
       p.gn_C = s0.C;
-      static const bool tanh32 = std::getenv("GP_PATCH_TANH32") != nullptr;     // A/B switch
-      p.gn_silu = a.gn_silu ? (tanh32 ? 2 : 1) : 0;
-      static const int xmode = std::getenv("GP_PATCH_XFORM") ? std::atoi(std::getenv("GP_PATCH_XFORM")) : 0;
-      p.gn_mode = xmode;
+      p.gn_silu = a.gn_silu ? 1 : 0;
     }
   }
   if (emit_stats) {
@@ -522,14 +506,13 @@ void Builder::attention_qkv(const std::string& name, const void* q, const void* 
   const int C = heads * d;
   const int PL = split_ ? 2 : 1;
   const long long TpP = (long long)Tp * PL;   // physical row pitch of S and V^T
-  static const bool unfused = std::getenv("GP_UNFUSED_ATTN") != nullptr;
   auto set_passes = [&](IgemmParams& p) {
     if (!split_) return;
     p.npass = 3;
     p.pass_amap[0] = 0; p.pass_amap[1] = 4; p.pass_amap[2] = 0;
     p.pass_bmap[0] = 0; p.pass_bmap[1] = 0; p.pass_bmap[2] = 1;
   };
-  if (d == 64 && !unfused && !split_) {   // fused tcgen05 flash-attention kernel (S and P stay on chip)
+  if (d == 64 && !split_) {   // fused tcgen05 flash-attention kernel (S and P stay on chip)
     if (measuring_) return;
     FattnParams p;
     std::memset(&p, 0, sizeof(p));

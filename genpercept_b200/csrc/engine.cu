@@ -454,14 +454,8 @@ struct gp_engine {
 
   // ------------------------------------------------------------------ graph pieces
   // 3x3 conv whose input is an NHWC8 tensor with `cin` (3 or 4) real channels: one 64-wide K chunk
-  // per tap through the tensor-core kernel (the TMA box zero-fills channels >= 8).  GP_DIRECT_SMALL=1
-  // routes it through the SIMT direct kernel instead (bring-up triage only).
+  // per tap through the tensor-core kernel (the TMA box zero-fills channels >= 8).
   void small_cin_conv(Builder& b, const std::string& key, const T4& src8, int cin, const T4& out) {
-    static const bool direct = std::getenv("GP_DIRECT_SMALL") != nullptr;
-    if (direct) {
-      b.direct(key, src8, cin, direct_w(key, cin), out, 0, nullptr, 0);
-      return;
-    }
     ConvArgs c;
     c.srcs = {src8};
     c.w = &conv_w(key, {cin});
@@ -1858,9 +1852,9 @@ gp_status gp_bench_conv(int dtype, int N, int H, int W, int Cin, int Cout, int k
     te.e.dev_allocs.push_back(x);
     te.e.dev_allocs.push_back(y);
     GP_CUDA(cudaMemset(x, 0, (size_t)N * H * W * Cin * 2));
-    // a scratch arena for the epilogue statistics (GP_BENCH_STATS=1); externals are addressed relative to it
+    // the plan allocates nothing from its arena, but externals are addressed relative to the arena's base
     void* scratch = nullptr;
-    GP_CUDA(cudaMalloc(&scratch, (size_t)N * 160 * Cout * 2 * sizeof(float) + (1 << 20)));
+    GP_CUDA(cudaMalloc(&scratch, 1 << 20));
     te.e.dev_allocs.push_back(scratch);
     Builder b(te.e.bf16, false, reinterpret_cast<uint8_t*>(scratch));
     ConvArgs c;
@@ -1868,16 +1862,6 @@ gp_status gp_bench_conv(int dtype, int N, int H, int W, int Cin, int Cout, int k
     c.ks = ks; c.mode = mode;
     c.w = (mode == 3) ? &te.e.conv_up_w("t") : &te.e.conv_w("t", {Cin});
     c.out = b.external(y, N, Ho, Wo, Cout);
-    if (std::getenv("GP_BENCH_STATS")) c.want_stats = true;      // epilogue experiments: also emit the GroupNorm partial sums
-    void* res = nullptr;
-    T4 rest;
-    if (std::getenv("GP_BENCH_RES")) {              // ... and / or add a residual of the output's shape
-      GP_CUDA(cudaMalloc(&res, (size_t)N * Ho * Wo * Cout * 2));
-      GP_CUDA(cudaMemset(res, 0, (size_t)N * Ho * Wo * Cout * 2));
-      te.e.dev_allocs.push_back(res);
-      rest = b.external(res, N, Ho, Wo, Cout);
-      c.res1 = &rest;
-    }
     b.conv("bench", c);
     cudaEvent_t e0, e1;
     GP_CUDA(cudaEventCreate(&e0));

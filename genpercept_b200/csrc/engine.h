@@ -74,7 +74,6 @@ class Arena {
   struct Blk { size_t off, size; bool free; };
   std::vector<Blk> blks_;
   size_t high_ = 0;
-  size_t nalloc_ = 0;
 };
 
 struct Op {

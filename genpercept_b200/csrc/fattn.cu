@@ -27,7 +27,6 @@
 
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "launch.h"
 #include "ptx.cuh"
@@ -51,17 +50,6 @@ __device__ __forceinline__ float ex2(float x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-// exp2 on the FMA pipe: round-to-nearest split x = n + f, |f| <= 0.5 (magic-number add), cubic minimax
-// 2^f (max relative error 7.5e-5, below the 16-bit rounding of P), n added into the exponent field.
-// Valid for x in [-126, 127].
-__device__ __forceinline__ float ex2_fma(float x) {
-  x = fmaxf(x, -126.f);
-  const float magic = 12582912.f;              // 1.5 * 2^23: the integer part lands in the low mantissa bits
-  const float r = x + magic;
-  const float f = x - (r - magic);
-  const float pl = fmaf(fmaf(fmaf(0.0551716685f, f, 0.242611125f), f, 0.693260968f), f, 0.999928057f);
-  return __int_as_float(__float_as_int(pl) + (__float_as_int(r) << 23));
-}
 template <bool BF16>
 __device__ __forceinline__ uint32_t pack16(float a, float b) {
   if constexpr (BF16) {
@@ -79,8 +67,7 @@ __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 
-// POLY: one exponential in four of the probability pass on the FMA pipe instead of the MUFU.
-template <bool BF16, bool POLY>
+template <bool BF16>
 __global__ void __launch_bounds__(kThreads, 1) fattn_kernel(const __grid_constant__ FattnParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -128,8 +115,6 @@ __global__ void __launch_bounds__(kThreads, 1) fattn_kernel(const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();      // see ptx.cuh: the next kernel may be scheduled; it blocks in its own pdl_wait
-  pdl_wait();         // set-up done; the predecessor grid has completed before any of its outputs is read
 
   if (warp == 8) {
     // ------------------------------------------------------------------ TMA producer (whole warp waits, one lane issues)
@@ -233,12 +218,8 @@ __global__ void __launch_bounds__(kThreads, 1) fattn_kernel(const __grid_constan
     // MUFU (2 x 128 x 8 cycles per sub-partition) and both idle it together during the rest of the block
     // (r1j: 3700 cycles per block).  With strict alternation (A_j, B_j, A_j+1, ...; two mbarriers) one
     // tile's load / max / wait phases run under the other's exponentials: 3200 cycles, 11.7 -> 9.8 ms
-    // per step.  `stagger` (a start offset for tile B) is the cheaper idea that did not hold the phase.
-    const bool pingpong = p.pingpong && ntile == 2;
-    if (t == 1 && p.stagger > 0) {
-      const long long t0 = clock64();
-      while (clock64() - t0 < p.stagger) {}
-    }
+    // per step.  A start offset for tile B is the cheaper idea that did not hold the phase.
+    const bool pingpong = ntile == 2;
     for (int j = 0; j < nblk; ++j) {
       if (tr && j < 64) p.trace[j * 8 + 0] = clock64();
       mbar_wait(&s_full[t], j & 1, 15);
@@ -307,11 +288,12 @@ __global__ void __launch_bounds__(kThreads, 1) fattn_kernel(const __grid_constan
 #pragma unroll
         for (int q = 0; q < 32; ++q) {
           const float x = __uint_as_float(s[c][q]) * c2 - mb;      // <= thr
-          pv[q] = (POLY && (q & 3) == 3) ? ex2_fma(x) : ex2(x);
+          pv[q] = ex2(x);
         }
-        // hand the MUFU to the other tile once the exponentials of chunk `pp_early` are issued: its wake-up latency
-        // and the first FFMAs of its pass run under this tile's remaining sums / packs / stores
-        if (pingpong && c == p.pp_early) mbar_arrive(&pp[1 - t]);
+        // hand the MUFU to the other tile once the exponentials of chunk 1 are issued: its wake-up latency and the first
+        // FFMAs of its pass run under this tile's remaining sums / packs / stores (r1l trace, block period in cycles by
+        // hand-over chunk: 3440 (0) / 3180 (1) / 3290 (2) / 3350 (3) / 3560 (after the pass))
+        if (pingpong && c == 1) mbar_arrive(&pp[1 - t]);
 #pragma unroll
         for (int q = 0; q < 32; q += 8) {
           l0 += pv[q]; l1 += pv[q + 1]; l2 += pv[q + 2]; l3 += pv[q + 3];
@@ -325,7 +307,6 @@ __global__ void __launch_bounds__(kThreads, 1) fattn_kernel(const __grid_constan
                        pack16<BF16>(pv[8 * i + 6], pv[8 * i + 7]));
       }
       l += ((l0 + l1) + (l2 + l3)) + ((l4 + l5) + (l6 + l7));
-      if (pingpong && p.pp_early >= 4) mbar_arrive(&pp[1 - t]);
       if (tr && j < 64) p.trace[j * 8 + 5] = clock64();
       tc_fence_before();                          // the O_t rescale (if any) is ordered before the next P.V
       fence_proxy_async_smem();                   // P_t visible to the tensor core (async proxy)
@@ -371,44 +352,23 @@ static long long* g_trace = nullptr;
 void fattn_set_trace(long long* dev_buf) { g_trace = dev_buf; }
 long long* fattn_get_trace() { return g_trace; }
 
-cudaError_t fattn_launch(const FattnParams& p_in, cudaStream_t stream) {
+cudaError_t fattn_launch(const FattnParams& p, cudaStream_t stream) {
   static bool attr_dev[64] = {};
-  static bool poly = false;
-  static int stagger = 0, pingpong = 1, pp_early = 1;   // r1l trace: period 3560 (4) / 3350 (3) / 3290 (2) / 3180 (1) / 3440 (0)
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
   bool& attr_set = attr_dev[dev];      // function attributes are per device
   if (!attr_set) {
-    const void* fns[4] = {(const void*)fattn_kernel<false, false>, (const void*)fattn_kernel<false, true>,
-                          (const void*)fattn_kernel<true, false>, (const void*)fattn_kernel<true, true>};
-    for (const void* f : fns) {
+    for (const void* f : {(const void*)fattn_kernel<false>, (const void*)fattn_kernel<true>}) {
       cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
       if (e != cudaSuccess) return e;
     }
-    const char* env = getenv("GP_FATTN_POLY");   // 1: a quarter of the exponentials on the FMA pipe (A/B switch)
-    if (env && env[0] == '1') poly = true;
-    env = getenv("GP_FATTN_STAGGER");            // cycles (experiment)
-    if (env) stagger = atoi(env);
-    env = getenv("GP_FATTN_PP");                 // 0: let the exponential passes of the two tiles overlap (A/B switch)
-    if (env && env[0] == '0') pingpong = 0;
-    env = getenv("GP_FATTN_PP_EARLY");           // 0..3: hand over after that 32-column chunk's exponentials; 4: after the pass
-    if (env) pp_early = atoi(env);
     attr_set = true;
   }
-  FattnParams p = p_in;
-  p.stagger = stagger;
-  p.pingpong = pingpong;
-  p.pp_early = pp_early;
   const int grid = p.B * p.heads * ((p.q_tiles + 1) / 2);
   if (grid <= 0) return cudaSuccess;
-  if (p.bf16) {
-    if (poly) launch(fattn_kernel<true, true>, grid, kThreads, kSmemBytes, stream, p);
-    else launch(fattn_kernel<true, false>, grid, kThreads, kSmemBytes, stream, p);
-  } else {
-    if (poly) launch(fattn_kernel<false, true>, grid, kThreads, kSmemBytes, stream, p);
-    else launch(fattn_kernel<false, false>, grid, kThreads, kSmemBytes, stream, p);
-  }
+  if (p.bf16) launch(fattn_kernel<true>, grid, kThreads, kSmemBytes, stream, p);
+  else launch(fattn_kernel<false>, grid, kThreads, kSmemBytes, stream, p);
   return cudaGetLastError();
 }
 

@@ -16,9 +16,6 @@ struct FattnParams {
   float scale_log2e;
   int bf16;
   long long* trace;   // debug: CTA 0 records clock64() at phase boundaries (null = off); see scripts/fattn_trace.py
-  int stagger;        // cycles the softmax warps of tile B wait before their first block (set by fattn_launch)
-  int pingpong;       // 1: the exponential passes of the two tiles strictly alternate (set by fattn_launch)
-  int pp_early;       // chunk (0..3) after whose exponentials the turn is handed over; 4 = after the whole pass
 };
 
 void fattn_set_trace(long long* dev_buf);   // applies to subsequently built FattnParams (debug only)

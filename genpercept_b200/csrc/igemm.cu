@@ -19,7 +19,6 @@
 // halves the weight traffic and the per-byte barrier / TMA issue cost of the narrow-N layers.
 #include "igemm.h"
 
-#include <cstdlib>
 #include <cstring>
 
 #include "igemm_common.cuh"
@@ -71,8 +70,6 @@ __global__ void __launch_bounds__(kTapThreads, 1) igemm_kernel(const __grid_cons
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();      // the next kernel of the stream may be scheduled (it blocks in its own pdl_wait until this grid is done)
-  pdl_wait();         // barriers / TMEM are set up; from here on the predecessor's outputs are read
 
   // Single-thread roles run warp-uniform (every lane walks the loop and waits on the barriers) and one
   // elected lane issues: the TMA coordinates / UMMA descriptors then stay in uniform registers.
@@ -178,12 +175,12 @@ __global__ void __launch_bounds__(kTapThreads, 1) igemm_kernel(const __grid_cons
     }
   } else if (warp < kEpiWarps && p.epi_warps == kEpiWarps) {
     if (p.tma_store) run_epilogue_staged<BF16, kEpiWarps, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-    else run_epilogue_direct<BF16, kEpiWarps>(p, sacc, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
+    else run_epilogue_direct<BF16, kEpiWarps>(p, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
   } else if (warp < 4) {
     // four epilogue warps (warps 4..7 idle): the long-K BN = 256 layers, where eight 4 KiB staging tiles would cost the fourth
     // pipeline stage (igemm_finalize) and the epilogue is hidden behind an 18 k-cycle main loop anyway
     if (p.tma_store) run_epilogue_staged<BF16, 4, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-    else run_epilogue_direct<BF16, 4>(p, sacc, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
+    else run_epilogue_direct<BF16, 4>(p, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
   }
 
   tc_fence_before();
@@ -285,12 +282,12 @@ const char* igemm_finalize(IgemmParams* p) {
   const int stats_bytes = p->stats ? 4 * p->Cout * 2 * (int)sizeof(float) : 0;
   if (p->tma_store && ((p->Cout % 64) || (p->BN % 64) || (p->flags & IG_OUT_F32_NCHW) || p->out_z0 != 0))
     return "staged epilogue needs Cout % 64 == 0, BN % 64 == 0, plain 16-bit NHWC output";
-  if (p->tma_store && (p->flags & IG_GEGLU) && ((p->Cout % 128) || (p->BN % 128))) return "staged GEGLU needs Cout, BN % 128 == 0";
+  if (p->tma_store && (p->flags & IG_GEGLU)) return "GEGLU needs the direct epilogue";
   if (p->stats && (!p->tma_store || p->Cout > 512 || (p->flags & IG_GEGLU))) return "statistics need the staged epilogue and Cout <= 512";
   // staging: one 4 KiB tile per epilogue warp (8; 4 in the patch kernel's GroupNorm-transform build), x2 for the (hi, lo) layout
   int epi_warps = (p->patch && p->gn_ss) ? 4 : 8;
   // patch-resident layers without a residual: four warps and the fourth 16 KiB weight-ring stage (see igemm_patch.cu, NE4)
-  if (p->patch && !p->gn_ss && p->tma_store && !p->res_tma && p->res1 == nullptr && p->res2 == nullptr && getenv("GP_PATCH_NE8") == nullptr)
+  if (p->patch && !p->gn_ss && p->tma_store && !p->res_tma && p->res1 == nullptr && p->res2 == nullptr)
     epi_warps = 4;
   auto staging_of = [&](int ew) { return p->tma_store ? ew * 4096 * (p->out_lo ? 2 : 1) : 0; };
   int nkb_max = 0;
@@ -298,7 +295,7 @@ const char* igemm_finalize(IgemmParams* p) {
   // Eight staging tiles + the statistics scratch leave the BN = 256 layers three 48 KiB stages instead of four (r2: the
   // 512- and 256-channel VAE convs ran 8-15 % slower than in round 1: 929 -> 1006..1069 us).  Their main loop is >= 16 K
   // blocks (18 k cycles per tile) and hides a four-warp epilogue, so those layers keep four warps and the fourth stage.
-  if (!p->patch && epi_warps == 8 && nkb_max >= 16 && getenv("GP_EPI_WARPS8") == nullptr &&
+  if (!p->patch && epi_warps == 8 && nkb_max >= 16 &&
       (kMaxSmem - 3072 - stats_bytes - staging_of(4)) / stage_bytes > (kMaxSmem - 3072 - stats_bytes - staging_of(8)) / stage_bytes)
     epi_warps = 4;
   p->epi_warps = epi_warps;
@@ -306,7 +303,7 @@ const char* igemm_finalize(IgemmParams* p) {
   // bias: one N tile (288 floats, inside the 3072 reserved bytes) or the whole padded vector when it is small (<= 16 KiB)
   p->bias_slots = kBiasSlots;
   p->bias_all = 0;
-  if (p->n_tiles_n > 1 && p->n_tiles_n * p->BN + 32 <= 4096 && getenv("GP_NO_BIAS_ALL") == nullptr) {
+  if (p->n_tiles_n > 1 && p->n_tiles_n * p->BN + 32 <= 4096) {
     p->bias_all = 1;
     p->bias_slots = p->n_tiles_n * p->BN + 32;
   }
@@ -331,10 +328,6 @@ const char* igemm_finalize(IgemmParams* p) {
       p->bias_all = 0;
       p->bias_slots = kBiasSlots;
       st = (kMaxSmem - 3072 - stats_bytes - staging - 2 * p->a_slot_bytes) / (p->BN * 128);
-    }
-    if (const char* env = getenv("GP_PATCH_STAGES")) {          // experiment: depth of the weight ring
-      const int v = atoi(env);
-      if (v >= 2 && v < st) st = v;
     }
   }
   if (st > 8) st = 8;

@@ -96,7 +96,6 @@ struct IgemmParams {
                                  // layer has several N tiles and Cout is small enough, all of them (loaded once: bias_all)
   int bias_all;
   int epi_warps;                 // epilogue warps of the tap-streaming kernel: 8, or 4 where 8 would cost a pipeline stage (igemm_finalize)
-  int res_prefetch;              // L2-prefetch the next tile's residual boxes one tile period ahead (GP_NO_RES_PREFETCH=1: off)
   CUtensorMap tmRes[kMaxClasses];
   // Patch-resident main loop (igemm_patch.cu; 3x3 stride-1, one source, TW = 128, TH = MT = 1 or 2): per
   // 64-channel K chunk ONE (TH+2) x (TW+2) halo patch is loaded and all nine taps are fed from it by
@@ -115,7 +114,6 @@ struct IgemmParams {
   const float* gn_ss;            // null: the source is used as it is
   int gn_C;                      // channels of the normalised tensor (= the patch source's)
   int gn_silu;
-  int gn_mode;                   // experiment switches of the transform loop (GP_PATCH_XFORM), see igemm_patch.cu
 };
 
 cudaError_t igemm_patch_launch(const IgemmParams& p, int grid, cudaStream_t stream);   // igemm_patch.cu

@@ -135,10 +135,10 @@ __device__ __forceinline__ void bias32(const float* sbias, int c, float (&bz)[32
 // Staged epilogue (shared by the tap-streaming and the patch-resident main loops): TMEM -> registers
 // (bias / residuals / ReLU) -> 16-bit rows in a SWIZZLE_128B shared tile -> one TMA store per
 // (warp, 64-channel group), plus the GroupNorm partial sums read back column-wise from the tile.
-// SPLIT / RES / GEGLU are compile-time: with run-time flags one 32 x 64 piece executed ~830 warp instructions, 97 of them MOVs
+// SPLIT / RES are compile-time: with run-time flags one 32 x 64 piece executed ~830 warp instructions, 97 of them MOVs
 // and 27 branches around the variants not taken (ncu source page, r2q: the 320 -> 2560 linear issues 13.4 k warp
 // instructions per 128 x 256 tile against 2560 tensor cycles).  RES: 0 none, 1 residual tile through TMA, 2 per-thread rows.
-template <bool BF16, int NW, bool SPLIT, int RES, bool GEGLU>
+template <bool BF16, int NW, bool SPLIT, int RES>
 __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* stg_base, float* sacc, float* sbias, uint64_t* tfull_bar,
                                                 uint64_t* tempty_bar, uint64_t* res_bar, uint32_t tmem_base, int warp, int lane) {
   // ===================================================================== epilogue, staged + TMA store
@@ -153,20 +153,19 @@ __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* s
   const uint32_t my_row = stg_addr + lane * 128;
   constexpr bool split = SPLIT;              // high-precision mode: a second staged tile (+NW * 4 KiB) takes the lo plane
   const uint32_t my_row_lo = my_row + NW * 4096;
-  // 64-channel groups (128 GEMM columns with GEGLU) of the N tile go to the two halves by parity; a tile with one group only
-  // is done by half 0 (statistics: the halves then never accumulate the same channel into sacc[wq])
-  constexpr int gshift = GEGLU ? 7 : 6;
-  const bool two_groups = NW == 8 && (p.BN >> gshift) >= 2;
-  auto mine = [&](int c0) { return NW == 4 || (two_groups ? ((c0 >> gshift) & 1) == half : half == 0); };
+  // 64-channel groups of the N tile go to the two halves by parity; a tile with one group only is done by half 0
+  // (statistics: the halves then never accumulate the same channel into sacc[wq])
+  const bool two_groups = NW == 8 && (p.BN >> 6) >= 2;
+  auto mine = [&](int c0) { return NW == 4 || (two_groups ? ((c0 >> 6) & 1) == half : half == 0); };
   const int sw = lane & 7;
   int acc = 0;
   uint32_t acc_phase = 0, res_phase = 0;
   const bool relu = (p.flags & IG_RELU) != 0;
-  constexpr bool geglu = GEGLU;
   const bool do_stats = p.stats != nullptr;
   const int etid = threadIdx.x;
   int cur_img = -1;
   int cur_nt = -1;
+  // sum the four warp-private accumulators in a fixed order, publish this CTA's slot, reset
   auto flush_stats = [&](int img) {
     epi_sync<NW>();
     float* dst = p.stats + ((long long)img * p.stats_slots + blockIdx.x) * p.Cout * 2;
@@ -196,7 +195,7 @@ __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* s
     // those loads sit serially in front of every 32 x 64 piece of the epilogue, and with DRAM latency (1.5 us under
     // load) four of them per warp outlast the main loop of the short-K (Cout = 128) layers (r2: residual convs 20-30 %
     // slower than plain ones; the main loop of a 128->128 tile is 6 us).
-    if (RES == 1 && p.res_prefetch && lane == 0 && tile + (int)gridDim.x < p.total_tiles) {
+    if (RES == 1 && lane == 0 && tile + (int)gridDim.x < p.total_tiles) {
       const TileCoord tn = decode_tile(p, tile + gridDim.x);
       const int ncls = p.cls_from_z0 ? tn.z0 : 0;
       for (int h = 0; h < p.MT; ++h) {
@@ -227,46 +226,6 @@ __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* s
         const int n0 = n_base + c0;
         if (n0 >= p.Cout) break;
         if (!mine(c0)) continue;
-        if constexpr (geglu) {   // 128 GEMM columns = 4 x [16 values | 16 gates] -> 64 outputs = one staged 128-byte row
-          if (c0 & 64) continue;
-          if (lane == 0) tma_store_wait_read0();
-          __syncwarp();
-#pragma unroll
-          for (int sub = 0; sub < 4; ++sub) {
-            const int ns = n0 + sub * 32;
-            float bz[32];
-            bias32(sbias, ns - bias_origin, bz);
-            if (!waited) {
-              mbar_wait(&tfull_bar[acc], acc_phase, 4);
-              tc_fence_after();
-              waited = true;
-            }
-            uint32_t r[32];
-            tmem_ld_32x32(taddr + c0 + sub * 32, r);
-            tmem_ld_wait();
-            float g[16];
-#pragma unroll
-            for (int q = 0; q < 16; ++q) {
-              const float a = __uint_as_float(r[q]) + bz[q], gt = __uint_as_float(r[16 + q]) + bz[16 + q];
-              g[q] = valid ? a * gelu_erf(gt) : 0.f;
-            }
-#pragma unroll
-            for (int i = 0; i < 2; ++i) {
-              const uint32_t a = my_row + (((sub * 2 + i) ^ sw) << 4);
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(pack16<BF16>(g[8 * i], g[8 * i + 1])),
-                           "r"(pack16<BF16>(g[8 * i + 2], g[8 * i + 3])), "r"(pack16<BF16>(g[8 * i + 4], g[8 * i + 5])),
-                           "r"(pack16<BF16>(g[8 * i + 6], g[8 * i + 7]))
-                           : "memory");
-            }
-          }
-          fence_proxy_async_shared();
-          __syncwarp();
-          if (lane == 0) {
-            tma_store_4d(&p.tmOut[cls], stg_addr, n0 >> 1, sx, sy, t.z1);
-            tma_store_commit();
-          }
-          continue;
-        } else {
         if (lane == 0) tma_store_wait_read0();                // the previous store has finished reading the tile
         __syncwarp();
         uint4 rt[8];                                          // this thread's residual row (64 channels), res_tma only
@@ -384,7 +343,6 @@ __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* s
           float* d = sacc + ((size_t)wq * p.Cout + n0 + 2 * lane) * 2;
           d[0] += s0; d[1] += q0; d[2] += s1; d[3] += q1;
         }
-        }   // !GEGLU
       }
     }
     if (!waited) {
@@ -401,25 +359,21 @@ __device__ __forceinline__ void epilogue_staged(const IgemmParams& p, uint8_t* s
 }
 
 
-// Run-time flags -> the specialised staged epilogue.  LEAN (the patch-resident kernel): no (hi, lo) layout, no GEGLU.
+// Run-time flags -> the specialised staged epilogue.  LEAN (the patch-resident kernel): no (hi, lo) layout.
 template <bool BF16, int NW, bool LEAN>
 __device__ __forceinline__ void run_epilogue_staged(const IgemmParams& p, uint8_t* stg_base, float* sacc, float* sbias, uint64_t* tfull_bar,
                                                     uint64_t* tempty_bar, uint64_t* res_bar, uint32_t tmem_base, int warp, int lane) {
   const int rm = p.res_tma ? 1 : ((p.res1 != nullptr || p.res2 != nullptr) ? 2 : 0);
   if constexpr (!LEAN) {
-    if (p.flags & IG_GEGLU) {
-      epilogue_staged<BF16, NW, false, 0, true>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-      return;
-    }
     if (p.out_lo != 0) {
-      if (rm == 2) epilogue_staged<BF16, NW, true, 2, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-      else epilogue_staged<BF16, NW, true, 0, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
+      if (rm == 2) epilogue_staged<BF16, NW, true, 2>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
+      else epilogue_staged<BF16, NW, true, 0>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
       return;
     }
   }
-  if (rm == 1) epilogue_staged<BF16, NW, false, 1, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-  else if (rm == 2) epilogue_staged<BF16, NW, false, 2, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-  else epilogue_staged<BF16, NW, false, 0, false>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
+  if (rm == 1) epilogue_staged<BF16, NW, false, 1>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
+  else if (rm == 2) epilogue_staged<BF16, NW, false, 2>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
+  else epilogue_staged<BF16, NW, false, 0>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
 }
 
 // Direct epilogue: TMEM -> registers (bias / residuals / ReLU / affine clamp / GEGLU) -> global stores straight from
@@ -427,7 +381,7 @@ __device__ __forceinline__ void run_epilogue_staged(const IgemmParams& p, uint8_
 // LEAN = the GEGLU projection of the default mode (full 32-column chunks, no residual, 16-bit output, no (hi, lo) planes): every
 // other variant is compiled out of its loop (same reasoning as the staged epilogue's template parameters).
 template <bool BF16, int NW, bool LEAN>
-__device__ __forceinline__ void epilogue_direct(const IgemmParams& p, float* sacc, float* sbias, uint64_t* tfull_bar, uint64_t* tempty_bar,
+__device__ __forceinline__ void epilogue_direct(const IgemmParams& p, float* sbias, uint64_t* tfull_bar, uint64_t* tempty_bar,
                                                 uint32_t tmem_base, int warp, int lane) {
   // ===================================================================== epilogue
   const int wq = warp & 3;                 // warp % 4 -> TMEM lanes [32*wq, 32*wq+32)
@@ -442,25 +396,8 @@ __device__ __forceinline__ void epilogue_direct(const IgemmParams& p, float* sac
   const void* const res1 = LEAN ? nullptr : p.res1;
   const void* const res2 = LEAN ? nullptr : p.res2;
   const long long out_lo = LEAN ? 0 : p.out_lo;
-  const bool do_stats = false;               // statistics are produced by the staged (TMA store) epilogue only
   const int etid = threadIdx.x;              // 0..127 among the epilogue threads
-  int cur_img = -1;
   int cur_nt = -1;
-  // sum the four warp-private accumulators in a fixed order, publish this CTA's slot, reset
-  auto flush_stats = [&](int img) {
-    epi_sync<NW>();
-    float* dst = p.stats + ((long long)img * p.stats_slots + blockIdx.x) * p.Cout * 2;
-    for (int i = etid; i < 2 * p.Cout; i += NW * 32) {
-      const float tot = (sacc[i] + sacc[2 * p.Cout + i]) + (sacc[4 * p.Cout + i] + sacc[6 * p.Cout + i]);
-      dst[i] = tot;
-      sacc[i] = 0.f; sacc[2 * p.Cout + i] = 0.f; sacc[4 * p.Cout + i] = 0.f; sacc[6 * p.Cout + i] = 0.f;
-    }
-    epi_sync<NW>();
-  };
-  if (do_stats) {
-    for (int i = etid; i < 8 * p.Cout; i += NW * 32) sacc[i] = 0.f;
-    epi_sync<NW>();
-  }
   if (p.bias_all) load_bias_tile<NW>(p, sbias, 0, etid);
   for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
     const TileCoord t = decode_tile(p, tile);
@@ -472,13 +409,6 @@ __device__ __forceinline__ void epilogue_direct(const IgemmParams& p, float* sac
       cur_nt = t.n_tile;
     }
     const int bias_origin = p.bias_all ? 0 : n_base;
-    if (do_stats) {
-      const int img = p.stats_hw ? (t.tx * p.TW) / p.stats_hw : t.z1;
-      if (img != cur_img) {
-        if (cur_img >= 0) flush_stats(cur_img);
-        cur_img = img;
-      }
-    }
     for (int h = 0; h < p.MT; ++h) {
       const int row = h * 128 + wq * 32 + lane;
       const int ti = row >> p.tw_shift, tj = row & (p.TW - 1);
@@ -607,16 +537,15 @@ __device__ __forceinline__ void epilogue_direct(const IgemmParams& p, float* sac
     acc ^= 1;
     if (acc == 0) acc_phase ^= 1;
   }
-  if (do_stats && cur_img >= 0) flush_stats(cur_img);
 }
 
 template <bool BF16, int NW>
-__device__ __forceinline__ void run_epilogue_direct(const IgemmParams& p, float* sacc, float* sbias, uint64_t* tfull_bar,
-                                                    uint64_t* tempty_bar, uint32_t tmem_base, int warp, int lane) {
+__device__ __forceinline__ void run_epilogue_direct(const IgemmParams& p, float* sbias, uint64_t* tfull_bar, uint64_t* tempty_bar,
+                                                    uint32_t tmem_base, int warp, int lane) {
   const bool lean = (p.flags & IG_GEGLU) && !(p.flags & (IG_OUT_F32_NCHW | IG_RELU | IG_AFFINE_CLAMP01)) && p.out_lo == 0 &&
                     p.res1 == nullptr && p.res2 == nullptr && (p.BN % 32) == 0 && (p.Cout % p.BN) == 0;
-  if (lean) epilogue_direct<BF16, NW, true>(p, sacc, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
-  else epilogue_direct<BF16, NW, false>(p, sacc, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
+  if (lean) epilogue_direct<BF16, NW, true>(p, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
+  else epilogue_direct<BF16, NW, false>(p, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
 }
 
 }  // namespace

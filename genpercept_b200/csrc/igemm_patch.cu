@@ -25,8 +25,6 @@
 // owns the TMEM allocation —, warp 11 weight producer (one TMA box per (chunk, tap)).  GroupNorm-transform build
 // (XFORM = true, GP_GN_FUSE=1): warps 0..3 epilogue, 4..7 the same roles, 8..11 operand transform (GroupNorm scale/shift +
 // SiLU in place); registers re-balanced with setmaxnreg.
-#include <cstdlib>
-
 #include "igemm_common.cuh"
 #include "launch.h"
 
@@ -114,14 +112,12 @@ __global__ void __launch_bounds__(kPatchThreads, 1) igemm_patch_kernel(const __g
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();      // see ptx.cuh: the next kernel may be scheduled; it blocks in its own pdl_wait
-  pdl_wait();         // set-up done; the predecessor grid has completed before any of its outputs is read
 
   if (warp < NE) {
     // ===================================================================== epilogue
     if constexpr (XFORM) setmaxnreg_inc<232>();
     if (p.tma_store) run_epilogue_staged<BF16, NE, true>(p, stg_base, sacc, sbias, tfull_bar, tempty_bar, res_bar, tmem_base, warp, lane);
-    else epilogue_direct<BF16, NE, false>(p, sacc, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
+    else epilogue_direct<BF16, NE, false>(p, sbias, tfull_bar, tempty_bar, tmem_base, warp, lane);
   } else if (rw < 4) {
     if constexpr (XFORM) setmaxnreg_dec<72>();
     if (rw == 0) {
@@ -252,7 +248,6 @@ __global__ void __launch_bounds__(kPatchThreads, 1) igemm_patch_kernel(const __g
     const int jlog = cpos ^ (rbase & 7);             // this thread's logical channel group (8 channels) in every chunk
     const bool do_gn = p.gn_ss != nullptr;
     const bool do_silu = p.gn_silu != 0;
-    const bool tanh32 = p.gn_silu == 2;              // A/B switch: tanh.approx.f32 instead of the f16x2 form
     int slot = 0;
     uint32_t phase = 0;
     int trace_n = 0;
@@ -265,7 +260,7 @@ __global__ void __launch_bounds__(kPatchThreads, 1) igemm_patch_kernel(const __g
         float sc[8], sh[8];
         if (xf) {                                    // fetched before the patch lands
           const float4* sp = reinterpret_cast<const float4*>(ssn + (kc * kBK + jlog * 8) * 2);
-          const float pre = (do_silu && !BF16 && !tanh32) ? 0.5f : 1.f;   // the fp16 SiLU form takes h = x / 2: folded into the affine
+          const float pre = (do_silu && !BF16) ? 0.5f : 1.f;   // the fp16 SiLU form takes h = x / 2: folded into the affine
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
             const float4 a = __ldg(sp + e);
@@ -277,34 +272,7 @@ __global__ void __launch_bounds__(kPatchThreads, 1) igemm_patch_kernel(const __g
         if (trx && tix < 60) p.trace[tix * 8 + 0] = clock64();
         mbar_wait(&a_full[slot * 4], phase, 8);
         if (trx && tix < 60) p.trace[tix * 8 + 1] = clock64();
-        if (!xf) {
-        } else if (p.gn_mode & 2) {                  // experiment: one row per iteration
-          const uint32_t base = smem_u32(smem + slot * p.a_slot_bytes) + cpos * 16;
-          int py = 0, px = rbase;
-          for (int r = rbase; r < prows; r += 16) {
-            const bool inside = px < kPW && (unsigned)(y0 + py) < (unsigned)p.gridH && (unsigned)(x0 + px) < (unsigned)p.gridW;
-            if (inside) {
-              const uint32_t addr = base + r * 128;
-              uint32_t w[4];
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]) : "r"(addr));
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                float a = fmaf(cvt16<BF16>((uint16_t)(w[e] & 0xFFFF)), sc[2 * e], sh[2 * e]);
-                float b = fmaf(cvt16<BF16>((uint16_t)(w[e] >> 16)), sc[2 * e + 1], sh[2 * e + 1]);
-                if (BF16 || tanh32) {
-                  if (do_silu) { a = silu_tanh(a); b = silu_tanh(b); }
-                  w[e] = pack16<BF16>(a, b);
-                } else {
-                  w[e] = do_silu ? silu_pair_f16(a, b) : pack16<BF16>(a, b);
-                }
-              }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
-            }
-            px += 16;
-            if (px >= kPP) { px -= kPP; ++py; }
-          }
-          fence_proxy_async_shared();
-        } else {
+        if (xf) {
           const uint32_t base = smem_u32(smem + slot * p.a_slot_bytes) + cpos * 16;
           int py = 0, px = rbase;                    // rbase < 16 < kPW
           for (int r = rbase; r < prows; r += 64) {  // four rows in flight per thread
@@ -327,7 +295,7 @@ __global__ void __launch_bounds__(kPatchThreads, 1) igemm_patch_kernel(const __g
               for (int e = 0; e < 4; ++e) {
                 float a = fmaf(cvt16<BF16>((uint16_t)(w[u][e] & 0xFFFF)), sc[2 * e], sh[2 * e]);
                 float b = fmaf(cvt16<BF16>((uint16_t)(w[u][e] >> 16)), sc[2 * e + 1], sh[2 * e + 1]);
-                if (BF16 || tanh32) {
+                if constexpr (BF16) {
                   if (do_silu) { a = silu_tanh(a); b = silu_tanh(b); }
                   w[u][e] = pack16<BF16>(a, b);
                 } else {

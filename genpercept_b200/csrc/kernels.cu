@@ -3,8 +3,6 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include "launch.h"
 #include "ptx.cuh"
 
@@ -99,8 +97,6 @@ __device__ __forceinline__ float warp_max(float v) {
 // ------------------------------------------------------------------------------ direct conv
 template <bool BF16>
 __global__ void direct_conv_kernel(const DirectConvParams p) {
-  pdl_trigger();
-  pdl_wait();
   const long long total = (long long)p.N * p.Ho * p.Wo * p.Cout;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
@@ -145,8 +141,6 @@ __global__ void direct_conv_kernel(const DirectConvParams p) {
 template <bool BF16>
 __global__ void gn_stats_kernel(const uint16_t* __restrict__ x, long long HW, int C, float* __restrict__ partial,
                                 int Ctot, int coff, int pix_per_block, int xs, int lo) {
-  pdl_trigger();
-  pdl_wait();
   extern __shared__ float sh[];   // [PIX][C][2]
   const int n = blockIdx.y;
   const int tid = threadIdx.y * blockDim.x + threadIdx.x;
@@ -197,8 +191,6 @@ __global__ void gn_stats_kernel(const uint16_t* __restrict__ x, long long HW, in
 __global__ void __launch_bounds__(256) gn_finalize_kernel(GnSrc s0, GnSrc s1, int nsrc, const float* __restrict__ gamma,
                                                           const float* __restrict__ beta, int N, int Ctot, int groups,
                                                           float inv_count, float eps, float* __restrict__ ss) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ float red[2][8];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int n = blockIdx.x / groups, g = blockIdx.x % groups;
@@ -240,8 +232,6 @@ template <bool BF16, bool SILU>
 __global__ void gn_apply_kernel(const uint16_t* __restrict__ x, long long HW, int C, const float* __restrict__ ss,
                                 int Ctot, int coff, uint16_t* __restrict__ y, int y_cstride, int pix_per_block, int xs,
                                 int lo_x, int lo_y) {
-  pdl_trigger();
-  pdl_wait();
   // blockDim = (C/8 channel vectors, PIX pixel lanes); grid = (pixel chunks, N).  The thread's 8
   // (scale, shift) pairs live in registers for its whole pixel strip.
   const int n = blockIdx.y;
@@ -297,8 +287,6 @@ template <bool BF16, int KV, int TOK>
 __global__ void __launch_bounds__(256) layernorm_kernel(const uint16_t* __restrict__ x, uint16_t* __restrict__ y, long long tokens,
                                                         int C, const float* __restrict__ gamma, const float* __restrict__ beta,
                                                         float eps, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const int lane = threadIdx.x & 31;
   const long long tok0 = ((long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * TOK;
   if (tok0 >= tokens) return;
@@ -365,8 +353,6 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const uint16_t* __restri
 constexpr int kSmMaxVec = 8;   // T <= 256 threads * 8 vec * 8 = 16384
 template <bool BF16>
 __global__ void softmax_rows_small_kernel(uint16_t* __restrict__ s, long long rows, int T, int Tp, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const int lane = threadIdx.x & 31;
   const long long r = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (r >= rows) return;
@@ -385,8 +371,6 @@ __global__ void softmax_rows_small_kernel(uint16_t* __restrict__ s, long long ro
 // VAE mid-block rows (T = 9216) then hold 24 values per thread instead of 64 (r1_final: 2.5 TB/s at low occupancy).
 template <bool BF16, int MV>
 __global__ void softmax_rows_kernel(uint16_t* __restrict__ s, int T, int Tp, int lo) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ float red[32];
   uint16_t* row = s + (long long)blockIdx.x * (lo ? 2 * Tp : Tp);
   const int nvec = T / 8;
@@ -442,8 +426,6 @@ constexpr int kSmPipeThreads = 384;
 constexpr int kSmPipeSlots = 3;
 template <bool BF16, int MV>
 __global__ void __launch_bounds__(kSmPipeThreads) softmax_rows_pipe_kernel(uint16_t* __restrict__ s, long long rows, int T, int Tp) {
-  pdl_trigger();
-  pdl_wait();
   extern __shared__ __align__(128) uint8_t sm_raw[];
   __shared__ float red[2][kSmPipeThreads / 32];
   __shared__ __align__(8) uint64_t full[kSmPipeSlots];
@@ -536,8 +518,6 @@ template <bool BF16, int KV, int TOK>
 __global__ void xattn2_kernel(const uint16_t* __restrict__ x, uint16_t* __restrict__ y, long long tokens, int C,
                               int heads, const float* __restrict__ U, const float* __restrict__ u0,
                               const float* __restrict__ M, const float* __restrict__ c0, float eps, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const int lane = threadIdx.x & 31;
   const long long tok0 = ((long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * TOK;
   if (tok0 >= tokens) return;
@@ -645,8 +625,6 @@ __global__ void __launch_bounds__(KV >= 5 ? 512 : 256) xattn2_smem_kernel(const 
                                                           int C, int heads, const float* __restrict__ U,
                                                           const float* __restrict__ u0, const float* __restrict__ M,
                                                           const float* __restrict__ c0, float eps, int lo) {
-  pdl_trigger();
-  pdl_wait();
   extern __shared__ __align__(16) float xa_sm[];
   float* sU = xa_sm;
   float* sM = sU + heads * C;
@@ -773,8 +751,6 @@ __global__ void __launch_bounds__(KV >= 5 ? 512 : 256) xattn2_smem_kernel(const 
 // ------------------------------------------------------------------------------ elementwise
 template <bool BF16>
 __global__ void geglu_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, long long total_vec, int C4) {
-  pdl_trigger();
-  pdl_wait();
   const int nvec = C4 / 8;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec;
        i += (long long)gridDim.x * blockDim.x) {
@@ -792,8 +768,6 @@ __global__ void geglu_kernel(const uint16_t* __restrict__ in, uint16_t* __restri
 template <bool BF16>
 __global__ void relu_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, long long total_vec, int nvec,
                             int lo) {
-  pdl_trigger();
-  pdl_wait();
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec;
        i += (long long)gridDim.x * blockDim.x) {
     const long long off = lo ? (i / nvec) * (2LL * lo) + (i % nvec) * 8 : i * 8;   // [pixel][hi C | lo C]
@@ -808,8 +782,6 @@ __global__ void relu_kernel(const uint16_t* __restrict__ in, uint16_t* __restric
 template <bool BF16>
 __global__ void bilinear_up2x_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, int N, int H, int W,
                                      int C, float sy, float sx, long long total_vec, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const int nvec = C / 8;
   const int Ho = 2 * H, Wo = 2 * W;
   const int xs = lo ? 2 * C : C;
@@ -840,8 +812,6 @@ __global__ void bilinear_up2x_kernel(const uint16_t* __restrict__ in, uint16_t* 
 template <bool BF16>
 __global__ void preprocess_kernel(const void* __restrict__ in, int kind, uint16_t* __restrict__ out, int N,
                                   long long HW, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)N * HW) return;
   const int n = (int)(i / HW);
@@ -864,8 +834,6 @@ __global__ void preprocess_kernel(const void* __restrict__ in, int kind, uint16_
 template <bool BF16>
 __global__ void preprocess_im2col_kernel(const void* __restrict__ in, int kind, uint16_t* __restrict__ out, int N, int H, int W,
                                          int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long HW = (long long)H * W;
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)N * HW) return;
@@ -909,14 +877,10 @@ __device__ __forceinline__ float ord2f(unsigned int u) {
   return __uint_as_float((u & 0x80000000u) ? (u & 0x7FFFFFFFu) : ~u);
 }
 __global__ void minmax_init_kernel(unsigned int* s, int N) {
-  pdl_trigger();
-  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < N) { s[2 * i] = 0xFFFFFFFFu; s[2 * i + 1] = 0u; }
 }
 __global__ void minmax_reduce_kernel(const float* __restrict__ x, long long HW, unsigned int* s) {
-  pdl_trigger();
-  pdl_wait();
   const int n = blockIdx.y;
   float mn = INFINITY, mx = -INFINITY;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (long long)gridDim.x * blockDim.x) {
@@ -927,8 +891,6 @@ __global__ void minmax_reduce_kernel(const float* __restrict__ x, long long HW, 
   if ((threadIdx.x & 31) == 0) { atomicMin(&s[2 * n], f2ord(mn)); atomicMax(&s[2 * n + 1], f2ord(mx)); }
 }
 __global__ void minmax_apply_kernel(float* __restrict__ x, long long HW, const unsigned int* __restrict__ s, float dmin, int zero_min) {
-  pdl_trigger();
-  pdl_wait();
   const int n = blockIdx.y;
   const float mn = zero_min ? 0.f : ord2f(s[2 * n]), mx = ord2f(s[2 * n + 1]);
   const float d = fmaxf(mx - mn, dmin);
@@ -1050,8 +1012,7 @@ cudaError_t softmax_rows(void* sio, long long rows, int T, int Tp, bool bf16, cu
     return cudaGetLastError();
   }
   if (T / 8 > 256 * kSmMaxVec) return cudaErrorInvalidValue;
-  static const bool no_pipe = [] { const char* e = getenv("GP_SOFTMAX_PIPE"); return e && e[0] == '0'; }();
-  if (!split && !no_pipe && T >= 2048 && T / 8 <= kSmPipeThreads * 6 && rows >= 1024) {
+  if (!split && T >= 2048 && T / 8 <= kSmPipeThreads * 6 && rows >= 1024) {
     const int slot_bytes = (T * 2 + 127) & ~127;
     const int smem = kSmPipeSlots * slot_bytes;
     if (smem <= 200 * 1024) {
@@ -1105,9 +1066,8 @@ cudaError_t xattn2(const void* x, void* y, long long tokens, int C, int heads, c
   if (C % 8 || C / 8 > 32 * kLnMaxVec) return cudaErrorInvalidValue;
   const int kv = (C / 8 + 31) / 32;
   cudaError_t e = cudaSuccess;
-  static const bool no_smem = [] { const char* v = getenv("GP_XATTN_SMEM"); return v && v[0] == '0'; }();
   const size_t smem = ((size_t)2 * heads * C + C + heads) * sizeof(float);
-  if (!no_smem && heads % kXaHB == 0 && C % 32 == 0 && smem <= 226 * 1024) {
+  if (heads % kXaHB == 0 && C % 32 == 0 && smem <= 226 * 1024) {
     static int sms[64] = {0};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1182,8 +1142,6 @@ namespace {
 // 16-bit NHWC8 (first `c` channels) -> fp32 NCHW [N, c, H, W]
 template <bool BF16>
 __global__ void nhwc8_to_nchw_kernel(const uint16_t* __restrict__ in, float* __restrict__ out, int N, long long HW, int c, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)N * HW) return;
   const int n = (int)(i / HW);
@@ -1199,8 +1157,6 @@ __global__ void nhwc8_to_nchw_kernel(const uint16_t* __restrict__ in, float* __r
 template <bool BF16>
 __global__ void nchw4_affine_to_nhwc8_kernel(const float* __restrict__ in, uint16_t* __restrict__ out, int N, long long HW,
                                              float pre, const float* __restrict__ m, const float* __restrict__ b, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)N * HW) return;
   const int n = (int)(i / HW);
@@ -1229,8 +1185,6 @@ namespace {
 template <bool BF16>
 __global__ void latent_pack_kernel(const uint16_t* __restrict__ lat, const uint16_t* __restrict__ smp, uint16_t* __restrict__ xin,
                                    long long npx, int in_ch, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= npx) return;
   const long long o = i * (lo ? 16 : 8);
@@ -1251,8 +1205,6 @@ __global__ void latent_pack_kernel(const uint16_t* __restrict__ lat, const uint1
 template <bool BF16>
 __global__ void ddim_step_kernel(const uint16_t* __restrict__ mo, uint16_t* __restrict__ smp, uint16_t* __restrict__ x0, long long npx,
                                  float c0, float c1, float c2, float c3, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= npx) return;
   const long long o = i * (lo ? 16 : 8);
@@ -1271,8 +1223,6 @@ __global__ void ddim_step_kernel(const uint16_t* __restrict__ mo, uint16_t* __re
 template <bool BF16>
 __global__ void latent_affine_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, long long npx, float pre,
                                      const float* __restrict__ mat, const float* __restrict__ bias, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= npx) return;
   const long long o = i * (lo ? 16 : 8);
@@ -1346,8 +1296,6 @@ namespace {
 // median (torch.median: the LOWER middle value for an even count) or mean.
 __global__ void ensemble_reduce_kernel(const float* __restrict__ d, int B, long long HW, const float* __restrict__ sc,
                                        const float* __restrict__ sh, int median, float* __restrict__ out) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= HW) return;
   float v[32];
@@ -1373,8 +1321,6 @@ cudaError_t ensemble_reduce(const float* d, int B, long long HW, const float* sc
 namespace {
 __global__ void nearest_resize_kernel(const uint4* __restrict__ in, uint4* __restrict__ out, int N, int H, int W, int OH,
                                       int OW, int nvec, float sy, float sx, long long total_vec) {
-  pdl_trigger();
-  pdl_wait();
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec;
        i += (long long)gridDim.x * blockDim.x) {
     const int v = (int)(i % nvec);
@@ -1392,8 +1338,6 @@ __global__ void nearest_resize_kernel(const uint4* __restrict__ in, uint4* __res
 namespace {
 template <bool BF16>
 __global__ void softmax_groups_kernel(uint16_t* __restrict__ x, long long rows, int ld, int groups, int n, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= rows * groups) return;
   uint16_t* p = x + (i / groups) * (lo ? 2 * ld : ld) + (i % groups) * n;
@@ -1419,8 +1363,6 @@ namespace {
 template <bool BF16>
 __global__ void bilinear_resize_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, int N, int H, int W, int OH,
                                        int OW, int C, float sy, float sx, long long total_vec, int lo) {
-  pdl_trigger();
-  pdl_wait();
   const int nvec = C / 8;
   const int xs = lo ? 2 * C : C;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec;

@@ -1,18 +1,11 @@
-// Kernel launch helper: cudaLaunchKernelEx, optionally with the programmatic-dependent-launch attribute (see ptx.cuh,
-// pdl_wait).  Opt-in (GP_PDL=1): measured in one call (r2m) it changed nothing at batch 8 (95.05 / 96.21 ms with, 94.98 ms
-// without) and cost 1-2 % at batch 1 (384^2 .. 1024^2: 8.99 / 10.65 / 15.68 / 26.71 ms with, 8.84 / 10.45 / 15.59 / 26.54 ms
-// without) — inside a CUDA graph the launch gaps are already ~1 us and the early-resident CTAs only add scheduling work.
+// Kernel launch helper: cudaLaunchKernelEx with a plain stream-ordered configuration.  No programmatic dependent launch:
+// measured in one call (r2m) it changed nothing at batch 8 (95.05 / 96.21 ms with, 94.98 ms without) and cost 1-2 % at
+// batch 1 (384^2 .. 1024^2: 8.99 / 10.65 / 15.68 / 26.71 ms with, 8.84 / 10.45 / 15.59 / 26.54 ms without) — inside a CUDA
+// graph the launch gaps are already ~1 us and the early-resident CTAs only add scheduling work.
 #pragma once
 #include <cuda_runtime.h>
 
-#include <cstdlib>
-
 namespace gp {
-
-inline bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("GP_PDL"); return e && e[0] == '1'; }();
-  return on;
-}
 
 template <typename... P, typename... A>
 inline cudaError_t launch(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, A&&... args) {
@@ -21,11 +14,6 @@ inline cudaError_t launch(void (*kernel)(P...), dim3 grid, dim3 block, size_t sm
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<P>(args)...);
 }
 

@@ -26,15 +26,6 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-// ---------------------------------------------------------------- programmatic dependent launch
-// With GP_PDL=1 every kernel of the step is launched with programmaticStreamSerialization (launch.h): it may become
-// resident while its predecessor in the stream is still running, does its set-up (barrier init, TMEM allocation,
-// tensor-map prefetch) and then blocks in pdl_wait() until the predecessor grid has completed and its writes are visible.
-// pdl_trigger() lets the NEXT kernel be scheduled as soon as every CTA of this one has started.  Both are no-ops for a
-// launch without the attribute (the default).  Rule: no global-memory access before pdl_wait(), on any path.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // ---------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
